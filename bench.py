@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Learner steps/sec on synthetic (T=20, B=4096, O=24, A=4, H=256) trajectories.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Own arm (default): one process per GPU (torchrun for N > 1), global batch B=4096 sharded
 B/N per rank ("scaling": "strong"), one all-reduce of [gradient | loss scalars] per step (done by the
@@ -20,6 +20,7 @@ from __future__ import annotations
 
 import argparse
 import json
+import math
 import os
 import statistics
 import subprocess
@@ -181,7 +182,7 @@ def run_reference_arm(args):
     if rank != 0:
         return
     os.environ["CUDA_VISIBLE_DEVICES"] = ""  # the reference picks its device at import (learner.py:13)
-    steps, warm = max(1, min(args.steps, 20)), max(1, min(args.warmup, 2))
+    steps, warm = args.steps, max(1, min(args.warmup, 2))
     cb = cpu_reference_numbers(warm, steps)
     emit(reference_line(args, cb, steps, warm))
 
@@ -417,6 +418,44 @@ def kernel_breakdown(eng, flush, iters=20, barrier=lambda: None):
     return out
 
 
+DUMP_LIMIT = 64 << 20  # bytes, all arrays of one --dump-outputs together
+
+
+def last_step_outputs(eng, scalars):
+    """What the last timed step hands its caller, as float32 / float64 numpy arrays: the logged loss
+    scalars, the V-trace targets and advantages of this rank's batch, the gradient of the step
+    (float64, before clipping) and both networks' parameters after the update."""
+    import numpy as np
+    import torch
+
+    eng.synchronize()
+    out = {"scalars": np.array([scalars[k] for k in ("value_fn_loss", "policy_loss", "policy_entropy", "total_loss",
+                                                     "batch_mean_reward")], np.float64),
+           "vs": eng.vs.cpu().numpy(), "pg_adv": eng.pg_adv.cpu().numpy()}
+    for g, sd in eng.state(torch.float32).items():
+        for k, v in sd.items():
+            out[f"params.{g}.{k}"] = v.numpy()
+    for g, sd in eng.grads().items():
+        for k, v in sd.items():
+            out[f"grad.{g}.{k}"] = v
+    assert sum(v.nbytes for v in out.values()) == dump_bytes(eng)  # the size checked before the run
+    return out
+
+
+def dump_bytes(eng) -> int:
+    """Size of last_step_outputs(eng): 5 float64 scalars, vs + pg_adv (float32), params (float32) + grad (float64)."""
+    n_params = sum(math.prod(shp) for _, _, _, shp in eng._segments())
+    return 8 * 5 + 4 * (eng.vs.numel() + eng.pg_adv.numel()) + (4 + 8) * n_params
+
+
+def dump_outputs(path, outputs):
+    import numpy as np
+
+    os.makedirs(path, exist_ok=True)
+    for name, v in outputs.items():
+        np.save(os.path.join(path, name + ".npy"), v)
+
+
 def run_own_arm(args):
     import torch
 
@@ -442,6 +481,8 @@ def run_own_arm(args):
     hp = hparams(w["B"])
     eng = LearnerEngine(w["T"], Bl, w["O"], w["A"], w["H"], w["H"], hp, global_batch=w["B"],
                         device=f"cuda:{local}", process_group=pg, use_graph=not args.no_graph)
+    if args.dump_outputs and dump_bytes(eng) > DUMP_LIMIT:
+        raise SystemExit(f"bench.py: --dump-outputs would write {dump_bytes(eng)} bytes, more than {DUMP_LIMIT}")
     params0 = synth.init_params(0, w["O"], w["A"], w["H"])
     batches = [synth.shard_batch(synth.make_batch(1 + i, w["T"], w["B"], w["O"], w["A"]), rank, world)
                for i in range(2)]
@@ -504,6 +545,7 @@ def run_own_arm(args):
     dev_ms = max_over_ranks(sum(a.elapsed_time(b) for a, b in evs))
     launches = eng.launches_per_step * args.steps
     scal_dev = eng.read_scalars()
+    outputs = last_step_outputs(eng, scal_dev) if args.dump_outputs and rank == 0 else None
 
     # ---------------- end to end through host buffers ----------------
     # software pipeline: the DMA of batch i+1 (copy stream) runs under the kernels of batch i;
@@ -680,11 +722,19 @@ def run_own_arm(args):
         line["e2e_learner"] = e2e_learner
     if cb:
         line["cpu_baseline"] = cb
+    if outputs:
+        dump_outputs(args.dump_outputs, outputs)
     emit(line)
     if world > 1:
         import torch.distributed as dist
 
         dist.destroy_process_group()
+
+
+def positive_int(s: str) -> int:
+    if int(s) < 1:
+        raise argparse.ArgumentTypeError(f"must be at least 1, got {s}")
+    return int(s)
 
 
 def main():
@@ -697,7 +747,7 @@ def main():
     sys.stdout = sys.stderr  # python-level prints (the reference learner is chatty) go to stderr too
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
+    ap.add_argument("--steps", type=positive_int, default=200, help="timed steps")
     ap.add_argument("--warmup", type=int, default=10)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--no-graph", action="store_true", help="eager launches instead of CUDA graphs")
@@ -706,7 +756,11 @@ def main():
     ap.add_argument("--no-parity", action="store_true", help="skip the first-step oracle check")
     ap.add_argument("--no-weak", action="store_true", help="N > 1: skip the weak-scaling measurement")
     ap.add_argument("--no-learner", action="store_true", help="skip the run through Learner + RingQueue + actor processes")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed (rank 0) as DIR/<name>.npy, to compare builds")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the b200 arm's timed steps")
     select_workload(args.config)
     if args.impl == "reference":
         run_reference_arm(args)

@@ -1,8 +1,8 @@
 """TEST INFRASTRUCTURE - generate tests/golden/*.npz by running the REAL reference.
 
-Run here (the authoring container), where /root/reference exists:
+Run where the reference is importable ($IMPALA_REFERENCE_DIR, or oracle/_ref from oracle/make_ref.py):
 
-    python -m oracle.gen_golden
+    python -m oracle.gen_golden [name ...]      (default: every case, and the actor trajectories)
 
 For every case below a seeded synthetic batch per update is converted to the
 reference wire format (lists of float64 tensors), pushed through the unmodified
@@ -11,7 +11,13 @@ numbers the reference exposes are recorded: the five TensorBoard scalars of ever
 update (`learner.py:217-240`) and both state_dicts after every update.  The
 per-element tensors the reference keeps in locals (`vt`, `pg_adv`, `learner.py:127-135`)
 and the raw gradients are taken from `oracle/cpu_learner_port.py`, after asserting
-that the port reproduces the reference's scalars and parameters to 1e-12.
+that the port reproduces the reference's scalars and parameters to 1e-12.  A case with
+`sample=N` keeps every file under 1 MB: of each parameter larger than N entries, the parameters
+after every update and the raw gradients are stored only at N seeded flat indices
+(`sample_<net>_<key>`).
+
+`reference_actor` records what the reference's own actor.py ships: it runs unmodified against
+the in-repo old-API CartPole and its trajectories are stored densely (float64, zero padded).
 """
 from __future__ import annotations
 
@@ -40,7 +46,7 @@ CASES = {
     "c3_small_ragged": dict(T=20, B=48, O=24, A=4, H_pi=256, H_v=256, ragged=True,
                             unit_reward=False, updates=2, hp={}),
     "c5_small_long": dict(T=100, B=16, O=64, A=4, H_pi=512, H_v=512, ragged=False,
-                          unit_reward=False, updates=1, hp={}),
+                          unit_reward=False, updates=1, hp={}, sample=2048),
     "odd_shapes_clip": dict(T=12, B=32, O=7, A=3, H_pi=40, H_v=24, ragged=True,
                             unit_reward=False, updates=2,
                             hp=dict(max_norm=0.05, rho_bar=0.7, c_bar=0.9, entropy_c=0.01,
@@ -87,12 +93,64 @@ def run_reference(case, batches, params, hp):
     return per_update, snaps
 
 
-def main():
+def reference_actor(out_dir, B=6, T=20, H=16):
+    """B trajectories of the reference's actor.py (CartPole, policy hidden H, max_timesteps T)."""
+    import queue
+
+    import torch
+
+    from oracle import cartpole_env
+
+    refload.load(env_factory=cartpole_env.make)
+    import actor as ref_actor
+    import models as ref_models
+    import utils as ref_utils
+
+    hp = ref_utils.Hyperparameters(**default_hparams(batch_size=B, max_timesteps=T, verbose=0)._asdict())
+    torch.manual_seed(0)
+    shared = ref_models.MlpPolicy(4, 2, H)
+
+    class FakeLearner:  # what actor.py touches: .completion.is_set() and .policy_weights
+        class completion:
+            calls = 0
+
+            @classmethod
+            def is_set(cls):
+                cls.calls += 1
+                return cls.calls > B
+
+        policy_weights = shared.state_dict()
+
+    q = queue.Queue()
+    ref_actor.Actor(1, hp, ref_models.MlpPolicy(4, 2, H), FakeLearner, q, ref_utils.Counter(0))._act()
+    trajs = [q.get_nowait() for _ in range(B)]
+    blob = dict(meta_torch_version=np.array(torch.__version__), lens=np.zeros(B, np.int32),
+                obs=np.zeros((T + 1, B, 4)), logits=np.zeros((T, B, 2)), actions=np.zeros((T, B), np.int64),
+                rewards=np.zeros((T, B)), done=np.zeros((T, B), bool))
+    for b, tr in enumerate(trajs):
+        L = len(tr.r)
+        blob["lens"][b] = L
+        blob["obs"][:L + 1, b] = torch.stack(tr.obs).numpy()
+        blob["logits"][:L, b] = torch.stack(tr.logits).detach().numpy()
+        blob["actions"][:L, b] = torch.cat(tr.a).numpy()
+        blob["rewards"][:L, b] = torch.stack(tr.r).numpy()
+        blob["done"][:L, b] = torch.stack(tr.d).numpy()
+    os.makedirs(os.path.join(out_dir, "reference_actor"), exist_ok=True)
+    path = os.path.join(out_dir, "reference_actor", "cartpole.npz")
+    np.savez_compressed(path, **blob)
+    print(f"reference_actor: lens {blob['lens'].tolist()} -> {path} ({os.path.getsize(path) / 1024:.0f} KiB)")
+
+
+def main(names):
     import torch
 
     out_dir = os.path.join(ROOT, "tests", "golden")
     os.makedirs(out_dir, exist_ok=True)
+    if not names or "reference_actor" in names:
+        reference_actor(out_dir)
     for name, case in CASES.items():
+        if names and name not in names:
+            continue
         seed = sum(map(ord, name)) % 1000
         hp = default_hparams(batch_size=case["B"], max_updates=case["updates"],
                              max_timesteps=case["T"], policy_hidden_dims=case["H_pi"],
@@ -110,9 +168,18 @@ def main():
         for k, v in hp._asdict().items():
             if isinstance(v, (int, float)) and not isinstance(v, bool):
                 blob[f"hp_{k}"] = np.array(v)
+        keep = {}  # (net, key) -> flat indices stored of the parameters after each update and the raw gradients
         for grp in ("policy", "value_fn"):
             for k in PKEYS:
                 blob[f"init_{grp}_{k}"] = params[grp][k]
+                n = params[grp][k].size
+                if case.get("sample") and n > case["sample"]:
+                    idx = np.sort(np.random.default_rng(seed).choice(n, case["sample"], replace=False))
+                    keep[grp, k] = blob[f"sample_{grp}_{k}"] = idx.astype(np.int32)
+
+        def stored(grp, k, arr):
+            return arr.reshape(-1)[keep[grp, k]] if (grp, k) in keep else arr
+
         worst = 0.0
         for u, batch in enumerate(batches):
             res = port.update(synth.to_trajectories(batch), keep_elements=True)
@@ -128,7 +195,7 @@ def main():
                     d = np.abs(st[grp][k] - ref_snaps[u][grp][k]).max()
                     worst = max(worst, float(d))
                     assert d <= 1e-12, (name, u, grp, k, d)
-                    blob[f"u{u}_{grp}_{k}"] = ref_snaps[u][grp][k]
+                    blob[f"u{u}_{grp}_{k}"] = stored(grp, k, ref_snaps[u][grp][k])
             T, B = case["T"], case["B"]
             vs = np.zeros((T + 1, B))
             pg = np.zeros((T, B))
@@ -139,7 +206,7 @@ def main():
             blob[f"u{u}_vs"] = vs
             blob[f"u{u}_pg_adv"] = pg
             for i, (grp, k) in enumerate([(g, k) for g in ("policy", "value_fn") for k in PKEYS]):
-                blob[f"u{u}_rawgrad_{grp}_{k}"] = res["raw_grads"][i].numpy()
+                blob[f"u{u}_rawgrad_{grp}_{k}"] = stored(grp, k, res["raw_grads"][i].numpy())
             for k, v in batch.items():
                 blob[f"u{u}_in_{k}"] = v
         path = os.path.join(out_dir, name + ".npz")
@@ -149,4 +216,4 @@ def main():
 
 
 if __name__ == "__main__":
-    main()
+    main(sys.argv[1:])

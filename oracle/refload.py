@@ -16,10 +16,9 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 
 
 def reference_dir():
-    """Where the unmodified reference modules can be imported from: $IMPALA_REFERENCE_DIR, the
-    checkout under /root/reference (authoring container), or the copy oracle/make_ref.py left under
-    oracle/_ref/ (git-ignored build output that travels to the GPU box)."""
-    for d in (os.environ.get("IMPALA_REFERENCE_DIR"), "/root/reference", os.path.join(_HERE, "_ref")):
+    """Where the unmodified reference modules can be imported from: $IMPALA_REFERENCE_DIR, or the
+    copy oracle/make_ref.py left under the git-ignored oracle/_ref/."""
+    for d in (os.environ.get("IMPALA_REFERENCE_DIR"), os.path.join(_HERE, "_ref")):
         if d and os.path.isfile(os.path.join(d, "learner.py")):
             return d
     return None
@@ -37,7 +36,7 @@ def load(env_factory=None):
     """
     ref_dir = reference_dir()
     if ref_dir is None:
-        raise RuntimeError("reference not found (no /root/reference and no oracle/_ref: run python -m oracle.make_ref)")
+        raise RuntimeError("reference not found (set IMPALA_REFERENCE_DIR or run python -m oracle.make_ref)")
     os.environ["CUDA_VISIBLE_DEVICES"] = ""
     if "torch" in sys.modules:
         import torch

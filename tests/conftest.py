@@ -56,6 +56,12 @@ class Golden:
         return {g: {k: self.z[f"u{u}_rawgrad_{g}_{k}"] for k in PKEYS}
                 for g in ("policy", "value_fn")}
 
+    def pick(self, g, k, arr):
+        """`arr`, a full parameter-shaped array, at the entries params_after / raw_grads hold for it:
+        the files of the large networks keep those at a seeded sample of flat indices only."""
+        name = f"sample_{g}_{k}"
+        return np.asarray(arr).reshape(-1)[self.z[name]] if name in self.z.files else arr
+
 
 @pytest.fixture(params=golden_names())
 def golden(request):

@@ -31,7 +31,7 @@ def main():
     sys.path.insert(0, ROOT)
     sys.path.insert(0, REF)
     if not os.path.isfile(os.path.join(REF, "train.py")):
-        print("oracle/_ref missing: run python -m oracle.make_ref where /root/reference exists")
+        print("oracle/_ref missing: run python -m oracle.make_ref (copies it from the reference checkout)")
         sys.exit(2)
     import torch
 

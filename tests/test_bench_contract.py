@@ -37,9 +37,18 @@ def test_reference_arm_line():
 
 
 @pytest.mark.gpu
-def test_own_arm_line():
-    """Default arm on cuda:0: contract keys, a dominant-kernel roofline, clocks, launch count."""
-    d = run_bench("--steps", "5", "--warmup", "3", "--no-cpu", timeout=600)
+def test_own_arm_line(tmp_path):
+    """Default arm on cuda:0: contract keys, a dominant-kernel roofline, clocks, launch count, and the
+    outputs of the last timed step under --dump-outputs."""
+    import numpy as np
+
+    d = run_bench("--steps", "5", "--warmup", "3", "--no-cpu", "--dump-outputs", str(tmp_path / "out"), timeout=600)
+    dumped = {f[:-4]: np.load(tmp_path / "out" / f) for f in os.listdir(tmp_path / "out")}
+    assert {"scalars", "vs", "pg_adv", "params.policy.model.0.weight", "grad.value_fn.model.3.bias"} <= set(dumped)
+    assert all(a.dtype in (np.float32, np.float64) for a in dumped.values())
+    assert sum(a.nbytes for a in dumped.values()) <= 64 << 20
+    assert dumped["scalars"][3] == d["loss"]["device_resident"]
+    assert dumped["vs"].shape == (d["config"]["T"] + 1, d["config"]["B"]) and np.isfinite(dumped["vs"]).all()
     assert (BASE_KEYS - {"cpu_baseline"}) | {"roofline", "clocks", "gpu_launches", "kernels"} <= set(d)
     assert d["n_gpus"] == 1 and d["steps"] == 5 and d["warmup"] >= 3 and d["value"] > 0
     assert abs(d["value"] * d["ms_per_step"] - 1e3) < 1e-6 * 1e3

@@ -15,7 +15,7 @@ pytestmark = pytest.mark.gpu
 @pytest.mark.parametrize("allreduce", ["peer", "peer-standalone", "nccl"])
 def test_two_rank_learner_matches_single_gpu(allreduce):
     if torch.cuda.device_count() < 2:
-        pytest.skip("needs at least 2 GPUs (run with gpurun --gpus 2)")
+        pytest.skip("needs at least 2 GPUs")
     with socket.socket() as s:
         s.bind(("127.0.0.1", 0))
         port = s.getsockname()[1]
@@ -37,7 +37,7 @@ def test_dp_learner_process_two_gpus(tmp_path, transport):
     real queue / ring, worker rank spawned by it, shards DMA'd per rank, weights compared with the
     real reference's (golden c1)."""
     if torch.cuda.device_count() < 2:
-        pytest.skip("needs at least 2 GPUs (run with gpurun --gpus 2)")
+        pytest.skip("needs at least 2 GPUs")
     script = os.path.join(os.path.dirname(__file__), "learner_process_check.py")
     res = subprocess.run([sys.executable, script, str(tmp_path / "logs"), transport, "2"], capture_output=True,
                          text=True, timeout=300)

@@ -15,7 +15,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 def test_unmodified_train_py_runs_against_the_b200_learner(tmp_path):
     if not os.path.isfile(os.path.join(ROOT, "oracle", "_ref", "train.py")):
         pytest.fail("oracle/_ref is missing: __graft_entry__.build() / python -m oracle.make_ref creates it "
-                    "where /root/reference exists, and it travels to the GPU box with the snapshot")
+                    "from the reference checkout (oracle/make_ref.py)")
     script = os.path.join(os.path.dirname(__file__), "reference_train_check.py")
     out = tmp_path / "logs"
     out.mkdir()

@@ -8,13 +8,12 @@ import pytest
 import torch
 
 from conftest import PKEYS, ROOT
-from oracle import refload
 from oracle.cpu_learner_port import CpuLearnerPort
 from oracle.impala_oracle import BatchedLearner
 from torched_impala_b200 import _cabi, synth
 from torched_impala_b200.learner import Learner, pack_trajectory
 from torched_impala_b200.models import MlpPolicy, MlpValueFn
-from torched_impala_b200.utils import Counter, default_hparams
+from torched_impala_b200.utils import Counter, Trajectory, default_hparams
 
 
 def empty_views(T, B, O, A):
@@ -95,39 +94,24 @@ def test_learner_surface_and_no_cpu_fallback(tmp_path):
         assert lrn.completion.is_set()
 
 
-@pytest.mark.skipif(not refload.available(), reason="needs /root/reference (authoring container only)")
 def test_unmodified_reference_actor_feeds_the_packer():
-    """The reference's own actor.py, run unmodified against the in-repo old-API CartPole, produces
-    trajectories that (a) the packer accepts and (b) give the same update whether they go
-    through the reference's per-trajectory path or through the packed dense batch."""
-    import cartpole_env
-
-    refload.load(env_factory=cartpole_env.make)
-    import actor as ref_actor  # /root/reference/actor.py
-    import models as ref_models
-    import utils as ref_utils
-
-    B, T = 6, 20
-    hp = ref_utils.Hyperparameters(**default_hparams(batch_size=B, max_timesteps=T, verbose=0)._asdict())
-    torch.manual_seed(0)
-    shared = ref_models.MlpPolicy(4, 2, 16)
-
-    class FakeLearner:  # what actor.py touches: .completion.is_set() and .policy_weights
-        class completion:
-            calls = 0
-
-            @classmethod
-            def is_set(cls):
-                cls.calls += 1
-                return cls.calls > B
-
-        policy_weights = shared.state_dict()
-
-    q = queue.Queue()
-    act = ref_actor.Actor(1, hp, ref_models.MlpPolicy(4, 2, 16), FakeLearner, q, ref_utils.Counter(0))
-    act._act()
-    trajs = [q.get_nowait() for _ in range(B)]
+    """Trajectories the reference's own actor.py produced, run unmodified against the in-repo old-API
+    CartPole (tests/golden/reference_actor/cartpole.npz, oracle/gen_golden.py), rebuilt in its wire
+    format: (a) the packer accepts them and (b) they give the same update whether they go through
+    the reference's per-trajectory path or through the packed dense batch."""
+    z = np.load(os.path.join(ROOT, "tests", "golden", "reference_actor", "cartpole.npz"))
+    T, B = z["rewards"].shape
+    hp = default_hparams(batch_size=B, max_timesteps=T, verbose=0)
+    trajs = []
+    for b, L in enumerate(z["lens"].tolist()):  # what actor.py appends per step: obs (O,) f64, a (1,) i64,
+        tr = Trajectory((1, b + 1))             # r () f64, d () bool, logits (A,) f64
+        tr.obs.append(torch.from_numpy(z["obs"][0, b]))
+        for t in range(L):
+            tr.add(torch.from_numpy(z["obs"][t + 1, b]), torch.from_numpy(z["actions"][t, b:b + 1]),
+                   torch.tensor(z["rewards"][t, b]), torch.tensor(z["done"][t, b]), torch.from_numpy(z["logits"][t, b]))
+        trajs.append(tr)
     assert all(1 <= len(t.r) <= T and len(t.obs) == len(t.r) + 1 for t in trajs)
+    assert all(t.d[-1] or len(t.r) == T for t in trajs) and not any(d for t in trajs for d in t.d[:-1])
     views = empty_views(T, B, 4, 2)
     for b, tr in enumerate(trajs):
         pack_trajectory(views, b, tr, T)
