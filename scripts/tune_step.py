@@ -1,6 +1,6 @@
 """Whole-step time (CUDA graph, L2 flushed, mean over many steps) under different environment settings:
-    python scripts/tune_step.py IMPALA_PAIR_W_BWD=100,115,127,140 [--config c4] [--steps 200]
-One fresh engine (= fresh graph capture, the split is baked in at capture) per value."""
+    python scripts/tune_step.py IMPALA_MLP_TC=0,1 [--config c4] [--steps 200]
+One fresh engine (= fresh graph capture, the kernel choice is baked in at capture) per value."""
 import os
 import sys
 

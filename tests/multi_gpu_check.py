@@ -1,12 +1,16 @@
 """torchrun target: N-rank sharded learner steps vs a single-rank full-batch run.
 
     python -m torch.distributed.run --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
-        tests/multi_gpu_check.py
+        tests/multi_gpu_check.py [--obs O] [--hidden H]
 
 Every rank takes its B/N slice, all ranks all-reduce [gradient | loss scalars] once per step and
 apply identical clip+Adam; rank 0 additionally replays the same batches on one GPU with the
 full batch and compares loss scalars and parameters (float32 sum order differs -> ~1e-6).
+The network shape picks the kernels: obs 24 / hidden 256 (default) runs the paired tensor-core
+backward, which pushes the gradient itself; obs 64 / hidden 512 runs the wide kernels, followed by
+the stand-alone push producer.
 """
+import argparse
 import os
 import sys
 
@@ -27,7 +31,11 @@ def main():
     rank, world, local = int(os.environ["RANK"]), int(os.environ["WORLD_SIZE"]), int(os.environ["LOCAL_RANK"])
     torch.cuda.set_device(local)
     dist.init_process_group("nccl", device_id=torch.device("cuda", local))
-    T, B, O, A, H = 20, 512, 24, 4, 256
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--obs", type=int, default=24)
+    ap.add_argument("--hidden", type=int, default=256)
+    args = ap.parse_args()
+    T, B, O, A, H = 20, 512, args.obs, 4, args.hidden
     hp = default_hparams(batch_size=B, max_timesteps=T)
     params = synth.init_params(3, O, A, H)
     batches = [synth.make_batch(10 + u, T, B, O, A, ragged=(u == 1)) for u in range(3)]

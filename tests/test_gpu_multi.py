@@ -1,6 +1,7 @@
 """GPU (>= 2 devices): the data-parallel learner equals the single-GPU full-batch learner and the
 float64 oracle, with the gradient exchange as a push over NVLink peer memory from the backward's
-tail (default), from the stand-alone producer kernel, and through NCCL."""
+tail (paired tensor-core kernels, obs 24 / hidden 256), from the stand-alone producer kernel (wide
+kernels, obs 64 / hidden 512: the c5 networks), and through NCCL."""
 import os
 import socket
 import subprocess
@@ -20,11 +21,11 @@ def test_two_rank_learner_matches_single_gpu(allreduce):
         s.bind(("127.0.0.1", 0))
         port = s.getsockname()[1]
     script = os.path.join(os.path.dirname(__file__), "multi_gpu_check.py")
+    shape = ["--obs", "64", "--hidden", "512"] if allreduce == "peer-standalone" else ["--obs", "24", "--hidden", "256"]
     res = subprocess.run([sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node=2",
-                          "--master-addr", "127.0.0.1", "--master-port", str(port), script],
+                          "--master-addr", "127.0.0.1", "--master-port", str(port), script, *shape],
                          capture_output=True, text=True, timeout=240,
-                         env=dict(os.environ, IMPALA_ALLREDUCE=allreduce.split("-")[0],
-                                  IMPALA_PUSH_FUSED="0" if allreduce == "peer-standalone" else "1"))
+                         env=dict(os.environ, IMPALA_ALLREDUCE=allreduce.split("-")[0]))
     assert res.returncode == 0, res.stdout[-3000:] + res.stderr[-3000:]
     assert "MULTI_GPU_OK" in res.stdout
     want = {"peer": "allreduce=peer(fused)", "peer-standalone": "allreduce=peer(standalone)", "nccl": "allreduce=nccl"}[allreduce]

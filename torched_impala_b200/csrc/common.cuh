@@ -79,62 +79,18 @@ __device__ __forceinline__ double warp_sum_f64(double x) {
     return x;
 }
 
-// ---- programmatic dependent launch (PDL): kernels 2..4 of a learner step are launched with the
-// programmatic-stream-serialization attribute and call pdl_wait() before the first access to
-// anything their predecessor produces.  No kernel triggers early (no griddepcontrol.launch_dependents):
-// the trigger is the implicit one at the exit of each predecessor CTA, i.e. every write of the
-// predecessor precedes it, so the successor's CTAs are merely pre-staged - they occupy SMs as the
-// predecessor's CTAs drain and run their own prologue (barrier init, TMEM allocation, weight
-// staging, optimizer-state loads) while the last predecessor CTAs finish - and pdl_wait()
-// returns once the predecessor grid is complete and flushed.  (An early trigger at kernel start
-// was measured first: the optimizer then read gradients the backward's reduction phase had not
-// written yet - tests/test_gpu_fullsize.py caught it - so the wait must not be relied on to cover
-// writes issued after a trigger.)  Inside a captured CUDA graph these launches become programmatic
-// edges.  Measured on the B200 (c4, 100 steps): 84.9 us per step with the attribute, 84.3 us without -
-// without an early trigger there is nothing left to overlap, so the attribute is OFF by default
-// (IMPALA_PDL=1 enables it; the waits are no-ops on plain launches).
-__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-
-// cluster_x > 1: launch as thread-block clusters of that many CTAs along x (grid.x a multiple of it).
-template <typename... KArgs, typename... Args>
-static inline cudaError_t impala_launch_ex(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem,
-                                           cudaStream_t st, bool dependent, bool cooperative, Args&&... args) {
-    return impala_launch_cl(kernel, grid, block, smem, st, dependent, cooperative, 1, static_cast<Args&&>(args)...);
-}
-
-template <typename... KArgs, typename... Args>
-static inline cudaError_t impala_launch_cl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem,
-                                           cudaStream_t st, bool dependent, bool cooperative, int cluster_x,
-                                           Args&&... args) {
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = grid, cfg.blockDim = block, cfg.dynamicSmemBytes = smem, cfg.stream = st;
-    cudaLaunchAttribute attr[3];
-    unsigned n = 0;
-    if (cluster_x > 1) {
-        attr[n].id = cudaLaunchAttributeClusterDimension;
-        attr[n].val.clusterDim.x = (unsigned)cluster_x, attr[n].val.clusterDim.y = 1, attr[n].val.clusterDim.z = 1;
-        ++n;
-    }
-    if (dependent && impala_env_int("IMPALA_PDL", 0) != 0) {
-        attr[n].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        attr[n].val.programmaticStreamSerializationAllowed = 1;
-        ++n;
-    }
-    if (cooperative) {
-        attr[n].id = cudaLaunchAttributeCooperative;
-        attr[n].val.cooperative = 1;
-        ++n;
-    }
-    cfg.attrs = attr, cfg.numAttrs = n;
-    return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
-}
-
-// cooperative: the kernel contains a grid-wide barrier - the launch then FAILS (instead of the barrier
+// For kernels that contain a grid-wide barrier: a cooperative launch FAILS (instead of the barrier
 // hanging) when the CTAs cannot all be resident, e.g. under an MPS SM limit or in a green context.
 template <typename... KArgs, typename... Args>
-static inline cudaError_t impala_launch(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem,
-                                        cudaStream_t st, bool dependent, Args&&... args) {
-    return impala_launch_ex(kernel, grid, block, smem, st, dependent, false, static_cast<Args&&>(args)...);
+static inline cudaError_t impala_launch_cooperative(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem,
+                                                    cudaStream_t st, Args&&... args) {
+    cudaLaunchConfig_t cfg{};
+    cfg.gridDim = grid, cfg.blockDim = block, cfg.dynamicSmemBytes = smem, cfg.stream = st;
+    cudaLaunchAttribute attr;
+    attr.id = cudaLaunchAttributeCooperative;
+    attr.val.cooperative = 1;
+    cfg.attrs = &attr, cfg.numAttrs = 1;
+    return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
 }
 
 // ---- push-model all-reduce over peer memory, LL ("low latency") format (protocol: see optim.cu)

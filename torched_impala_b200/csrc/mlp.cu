@@ -158,14 +158,18 @@ int impala_mlp_launch(void (*kernel)(MlpArgs), const MlpArgs& a, const MlpConfig
     return impala_launch_status();
 }
 
+// GEMM-shaped layers go to the tensor cores (IMPALA_MLP_TC=0 forces the FP32 kernels).
+static bool tc_enabled() {
+    const char* tc_env = std::getenv("IMPALA_MLP_TC");
+    return !(tc_env && tc_env[0] == '0');
+}
+
 extern "C" int impala_mlp_forward(const float* x, const float* params, float* out, int M, int O,
                                   int H, int N2, void* stream) {
     if (!x || !params || !out) return IMPALA_ERR_BAD_ARG;
-    // GEMM-shaped layers go to the tensor cores (IMPALA_MLP_TC=0 forces the FP32 kernels).
-    const char* tc_env = std::getenv("IMPALA_MLP_TC");
-    if (!(tc_env && tc_env[0] == '0') && impala_mlp_fwd_tc_eligible(x, M, O, H, N2))
+    if (tc_enabled() && impala_mlp_fwd_tc_eligible(x, M, O, H, N2))
         return impala_mlp_fwd_tc(x, params, out, M, O, H, N2, (cudaStream_t)stream);
-    if (!(tc_env && tc_env[0] == '0') && impala_mlp_tcw_eligible(x, M, O, H, N2))
+    if (tc_enabled() && impala_mlp_tcw_eligible(x, M, O, H, N2))
         return impala_mlp_fwd_tcw(x, params, out, M, O, H, N2, (cudaStream_t)stream);
     MlpArgs a{};
     MlpConfig c{};
@@ -176,17 +180,11 @@ extern "C" int impala_mlp_forward(const float* x, const float* params, float* ou
     return dispatch(false, a, c, smem, (cudaStream_t)stream, &grid);
 }
 
-static bool pair_enabled() {
-    const char* tc_env = std::getenv("IMPALA_MLP_TC");
-    const char* pr_env = std::getenv("IMPALA_MLP_PAIR");
-    return !(tc_env && tc_env[0] == '0') && !(pr_env && pr_env[0] == '0');
-}
-
 extern "C" int impala_mlp_forward_pair(const float* x, const float* params_pi, const float* params_vf,
                                        float* logits, float* values, int M_pi, int M_vf, int O,
                                        int H_pi, int H_vf, int A, void* stream) {
     if (!x || !params_pi || !params_vf || !logits || !values) return IMPALA_ERR_BAD_ARG;
-    if (pair_enabled() && A >= 2 && A <= 4 && impala_mlp_fwd_tc_eligible(x, M_pi, O, H_pi, A) &&
+    if (tc_enabled() && A >= 2 && A <= 4 && impala_mlp_fwd_tc_eligible(x, M_pi, O, H_pi, A) &&
         impala_mlp_fwd_tc_eligible(x, M_vf, O, H_vf, 1))
         return impala_mlp_fwd_tc_pair(x, params_pi, params_vf, logits, values, M_pi, M_vf, O, H_pi, H_vf, A,
                                       (cudaStream_t)stream);
@@ -217,12 +215,11 @@ extern "C" int impala_mlp_backward(const float* x, const float* params, const fl
     a.x = x, a.params = params, a.dout = dout;
     a.ws = reinterpret_cast<float*>(static_cast<char*>(workspace) + kWsHeader);
     int grid = 0;
-    const char* tc_env = std::getenv("IMPALA_MLP_TC");
-    if (!(tc_env && tc_env[0] == '0') && impala_mlp_bwd_tc_eligible(x, dout, M, O, H, N2) &&
+    if (tc_enabled() && impala_mlp_bwd_tc_eligible(x, dout, M, O, H, N2) &&
         (reinterpret_cast<uintptr_t>(grad) & 15) == 0)
         return impala_mlp_bwd_tc(x, params, dout, a.ws, grad, static_cast<unsigned int*>(workspace), M, O, H,
                                  N2, (cudaStream_t)stream);  // reduces in-kernel
-    const bool wide = !(tc_env && tc_env[0] == '0') && impala_mlp_tcw_eligible(x, M, O, H, N2);
+    const bool wide = tc_enabled() && impala_mlp_tcw_eligible(x, M, O, H, N2);
     const int rc = wide ? impala_mlp_bwd_tcw(x, params, dout, a.ws, M, O, H, N2, (cudaStream_t)stream, &grid)
                         : dispatch(true, a, c, smem, (cudaStream_t)stream, &grid);
     if (rc != IMPALA_OK) return rc;
@@ -240,7 +237,7 @@ extern "C" int impala_mlp_backward_pair(const float* x, const float* params_pi, 
     if (!x || !params_pi || !params_vf || !dlogits || !dv || !grad_pi || !grad_vf || !workspace_pi ||
         !workspace_vf)
         return IMPALA_ERR_BAD_ARG;
-    if (pair_enabled() && A >= 2 && A <= 4 && impala_mlp_bwd_tc_eligible(x, dlogits, M_pi, O, H_pi, A) &&
+    if (tc_enabled() && A >= 2 && A <= 4 && impala_mlp_bwd_tc_eligible(x, dlogits, M_pi, O, H_pi, A) &&
         impala_mlp_bwd_tc_eligible(x, dv, M_vf, O, H_vf, 1) &&
         ((reinterpret_cast<uintptr_t>(grad_pi) | reinterpret_cast<uintptr_t>(grad_vf)) & 15) == 0) {
         const int64_t need_pi = impala_mlp_backward_workspace(M_pi, O, H_pi, A);
@@ -263,7 +260,7 @@ extern "C" int impala_mlp_backward_pair(const float* x, const float* params_pi, 
 // ---- data-parallel learner: the paired backward that pushes its result to the peers (optim.cu)
 extern "C" int impala_mlp_backward_pair_push_supported(int M_pi, int M_vf, int O, int H_pi, int H_vf, int A) {
     alignas(16) static const float probe[4] = {0.f, 0.f, 0.f, 0.f};  // alignment stand-in for the data pointers
-    return pair_enabled() && A >= 2 && A <= 4 && impala_mlp_bwd_tc_eligible(probe, probe, M_pi, O, H_pi, A) &&
+    return tc_enabled() && A >= 2 && A <= 4 && impala_mlp_bwd_tc_eligible(probe, probe, M_pi, O, H_pi, A) &&
            impala_mlp_bwd_tc_eligible(probe, probe, M_vf, O, H_vf, 1) &&
            (M_pi + 63) / 64 + (M_vf + 63) / 64 >= 2;
 }

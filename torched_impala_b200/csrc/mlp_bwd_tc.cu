@@ -157,16 +157,11 @@ __device__ __forceinline__ uint8_t* bwd_tc_body(const BwdTcArgs& a, const int ct
             tc::bulk_g2s(dst + kRawDzOffset, a.dout + row0 * a.N2, bytes_z, &bars->raw_full[rs]);
         }
     };
-    // Everything up to here - and the W1' staging / TMEM allocation below - only touches parameters
-    // and this kernel's own state; dout (dlogits / dv) is the V-trace kernel's output: the thread
-    // that issues the bulk copies waits for it now, everybody else after staging (PDL, common.cuh).
-    if (warp == 16 && lane == 0) {
-        pdl_wait();
+    // the first bulk copies are in flight while the W1' tiles are staged
+    if (warp == 16 && lane == 0)
         for (int i = 0; i < n_my && i < kRawStages; ++i) issue_raw(i);
-    }
     if (warp == 18) tc::tmem_alloc(&bars->tmem_base, 512);
     tc::stage_w1_tiles(w_hi, w_lo, W1, b1, H, O, tid, kThreads, /*bias_column=*/true);
-    pdl_wait();
     tc::fence_proxy_async();
     tc::tc_fence_before();
     __syncthreads();
@@ -665,7 +660,7 @@ int impala_mlp_bwd_tc(const float* x, const float* params, const float* dout, fl
     }
     int grid = a.num_tiles < sms ? a.num_tiles : sms;  // <= SM count: the grid barrier needs residency
     if (grid > kMaxParts) grid = kMaxParts;
-    if ((e = impala_launch_ex(kernel, grid, kThreads, kSmemBytes, st, true, true, a)) != cudaSuccess) return (int)e;
+    if ((e = impala_launch_cooperative(kernel, grid, kThreads, kSmemBytes, st, a)) != cudaSuccess) return (int)e;
     return impala_launch_status();
 }
 
@@ -694,14 +689,16 @@ int impala_mlp_bwd_tc_pair(const float* x, const float* params_pi, const float* 
     int grid = total_tiles < sms ? total_tiles : sms;
     if (grid > kMaxParts) grid = kMaxParts;
     if (grid < 2) return IMPALA_ERR_UNSUPPORTED_SHAPE;
+    // per-tile cost of a policy tile in % of a value-function tile, per 128 hidden units: measured on a B200 (c4)
+    constexpr int kPairCostBwd = 105;
     const int n_pi = impala_pair_split(a_pi.num_tiles, a_vf.num_tiles, grid,
-                                       impala_env_int("IMPALA_PAIR_W_BWD", 105) * (H_pi / 128),
+                                       kPairCostBwd * (H_pi / 128),
                                        100 * (H_vf / 128));
     // cooperative launch: the in-kernel grid barrier needs every CTA resident (ADVICE r1)
-    e = push ? impala_launch_ex(mlp_bwd_tc_pair_kernel<true>, grid, kThreads, kSmemBytes, st, true, true, a_pi, a_vf, n_pi, *push,
-                                extra, n_extra)
-             : impala_launch_ex(mlp_bwd_tc_pair_kernel<false>, grid, kThreads, kSmemBytes, st, true, true, a_pi, a_vf, n_pi,
-                                PushArgs{}, (const double*)nullptr, 0);
+    e = push ? impala_launch_cooperative(mlp_bwd_tc_pair_kernel<true>, grid, kThreads, kSmemBytes, st, a_pi, a_vf, n_pi,
+                                         *push, extra, n_extra)
+             : impala_launch_cooperative(mlp_bwd_tc_pair_kernel<false>, grid, kThreads, kSmemBytes, st, a_pi, a_vf, n_pi,
+                                         PushArgs{}, (const double*)nullptr, 0);
     if (e != cudaSuccess) return (int)e;
     return impala_launch_status();
 }

@@ -45,13 +45,12 @@ clip_adam_kernel(float* __restrict__ params, const double* __restrict__ grad, fl
     float pk[kKeep], mk[kKeep], vk[kKeep];
     double ss0 = 0.0, ss1 = 0.0;
 #pragma unroll
-    for (int k = 0; k < kKeep; ++k) {  // optimizer state: not touched by the backward, loaded before the wait
+    for (int k = 0; k < kKeep; ++k) {
         const int64_t i = first + k * stride;
         pk[k] = i < n_total ? params[i] : 0.f;
         mk[k] = i < n_total ? m[i] : 0.f;
         vk[k] = i < n_total ? v[i] : 0.f;
     }
-    pdl_wait();  // the gradient comes from the backward kernel
 #pragma unroll
     for (int k = 0; k < kKeep; ++k) {
         const int64_t i = first + k * stride;
@@ -158,7 +157,6 @@ constexpr int kPushThreads = 256;  // remote stores are credit-limited per SM: s
 // Stand-alone producer: local[0, n) -> slot `rank` of every rank's gather buffer.
 __global__ void __launch_bounds__(kPushThreads)
 peer_push_kernel(const double* __restrict__ local, int64_t n, PushArgs p) {
-    pdl_wait();  // `local` comes from the backward kernel
     const long long step = *p.seq + 1;
     const int64_t off = (step & 1) * p.buf_stride + (int64_t)p.rank * p.slot_stride;
     for (int64_t i = (int64_t)blockIdx.x * kPushThreads + threadIdx.x; i < n; i += (int64_t)gridDim.x * kPushThreads) {
@@ -208,7 +206,6 @@ gather_clip_adam_kernel(float* __restrict__ params, double* __restrict__ reduced
         s_bias[0] = (float)((double)lr / (1.0 - s_pow[0]));
         s_bias[1] = (float)(1.0 / sqrt(1.0 - s_pow[1]));
     }
-    pdl_wait();  // orders this kernel behind the local backward (its successors rely on that)
     const long long step64 = *seq + 1;
     const unsigned step = (unsigned)step64;
     __syncthreads();
@@ -323,9 +320,8 @@ extern "C" int impala_clip_adam(float* params, const double* grad, float* m, flo
                                 void* stream) {
     if (!params || !grad || !m || !v || !state) return IMPALA_ERR_BAD_ARG;
     if (n_total < 1 || n_policy < 0 || n_policy > n_total) return IMPALA_ERR_BAD_ARG;
-    const cudaError_t e = impala_launch(clip_adam_kernel, kAdamCluster, kAdamThreads, 0, (cudaStream_t)stream, true, params,
-                                        grad, m, v, state, n_policy, n_total, max_norm, lr, beta1, beta2, eps, norms_out);
-    if (e != cudaSuccess) return (int)e;
+    clip_adam_kernel<<<kAdamCluster, kAdamThreads, 0, (cudaStream_t)stream>>>(params, grad, m, v, state, n_policy, n_total,
+                                                                              max_norm, lr, beta1, beta2, eps, norms_out);
     return impala_launch_status();
 }
 
@@ -340,8 +336,7 @@ extern "C" int impala_peer_push(const double* local, int64_t n, void* const* pee
     if (e != cudaSuccess) return (int)e;
     int grid = (int)((n + kPushThreads - 1) / kPushThreads);
     if (grid > sms) grid = sms;
-    e = impala_launch(peer_push_kernel, grid, kPushThreads, 0, (cudaStream_t)stream, true, local, n, p);
-    if (e != cudaSuccess) return (int)e;
+    peer_push_kernel<<<grid, kPushThreads, 0, (cudaStream_t)stream>>>(local, n, p);
     return impala_launch_status();
 }
 
@@ -357,10 +352,8 @@ extern "C" int impala_gather_clip_adam(float* params, double* reduced, const voi
     if (reinterpret_cast<uintptr_t>(gather) & 15) return IMPALA_ERR_BAD_ARG;
     const unsigned long long timeout_ns =
         timeout_s > 0 ? (unsigned long long)(timeout_s * 1e9) : 600ull * 1000000000ull;
-    const cudaError_t e = impala_launch(gather_clip_adam_kernel, kAdamCluster, kAdamThreads, 0, (cudaStream_t)stream, true,
-                                        params, reduced, static_cast<const ulonglong2*>(gather), seq, slot_stride, buf_stride,
-                                        world, n_extra, m, v, state, n_policy, n_total, max_norm, lr, beta1, beta2, eps,
-                                        norms_out, err, timeout_ns);
-    if (e != cudaSuccess) return (int)e;
+    gather_clip_adam_kernel<<<kAdamCluster, kAdamThreads, 0, (cudaStream_t)stream>>>(
+        params, reduced, static_cast<const ulonglong2*>(gather), seq, slot_stride, buf_stride, world, n_extra, m, v, state,
+        n_policy, n_total, max_norm, lr, beta1, beta2, eps, norms_out, err, timeout_ns);
     return impala_launch_status();
 }

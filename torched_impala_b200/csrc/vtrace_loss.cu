@@ -17,14 +17,9 @@
 //   acc_i   = delta_i + disc_i c_i (acc_{i+1} - v_{i+1})          learner.py:130
 //   vs = acc + v (:131);  pg_t = rho_t (r_t + disc_t vs_{t+1} - v_t)   (:135)
 // i.e. the affine map F_i(x) = (delta_i - g_i v_{i+1}) + g_i x with g_i = disc_i c_i.
-#include <cooperative_groups.h>
 #include <math.h>
 
-#include <cstdlib>
-
 #include "common.cuh"
-
-namespace cg = cooperative_groups;
 
 namespace {
 
@@ -125,27 +120,18 @@ __device__ __forceinline__ void store_logits(float* __restrict__ p, unsigned ele
 // Total threads = B * NSEG, so the small benchmark batch (T = 20, B = 4096) still spreads over
 // 1280 warps and the long unroll (T = 100, B = 8192) keeps ~2 500 warps x S rows of loads in flight.
 // ------------------------------------------------------------------------------------------------
-template <int AP, int S, int MAXT, int MINB, bool WITH_LOSS, bool VEC>
-__global__ void __launch_bounds__(MAXT, MINB) vtrace_lane_kernel(const VtArgs a) {
+template <int AP, int S, bool WITH_LOSS, bool VEC>
+__global__ void __launch_bounds__(512, 1) vtrace_lane_kernel(const VtArgs a) {
     __shared__ float2 s_map[2][kMaxSeg][32];
-    __shared__ float2 s_cta[2][32];  // this CTA's segments composed into one map (read by the cluster)
     __shared__ double s_red[kMaxSeg][4];
-    pdl_wait();  // logits / values come from the forward kernel
-    // Long unrolls: the time segments of a trajectory group are spread over a thread-block CLUSTER
-    // (csize CTAs x nw warps x S steps per chunk - T = 100 fits ONE chunk of 8 x 7 x 2 steps), so a
-    // thread's critical path is one load -> math -> exchange -> fix-up -> store sequence instead of
-    // T / (S nw) of them back to back; the CTA-level maps travel through distributed shared memory.
-    cg::cluster_group cluster = cg::this_cluster();
-    const int csize = (int)cluster.num_blocks(), crank = (int)cluster.block_rank();
     const int lane = threadIdx.x & 31, w = threadIdx.x >> 5, nw = blockDim.x >> 5;
-    const int nseg = nw * csize, seg = crank * nw + w;  // segments per chunk, this thread's segment
     const int T = a.T, B = a.B, A = VEC ? AP : a.A;
-    const int b = (blockIdx.x / csize) * 32 + lane;
+    const int b = blockIdx.x * 32 + lane;
     const bool live = b < B;
     const int bl = live ? b : B - 1;  // column this lane loads
     const int L = live ? min(max(__ldg(a.lens + bl), 0), T) : 0;
     const float v0 = __ldg(a.v + bl);  // V(x_0): the reference's v[:1]
-    const int rows = S * nseg;
+    const int rows = S * nw;
     const int nch = (T + rows - 1) / rows;
     const bool ref_mode = a.mode == IMPALA_MODE_REFERENCE;
 
@@ -160,7 +146,7 @@ __global__ void __launch_bounds__(MAXT, MINB) vtrace_lane_kernel(const VtArgs a)
         unsigned char dn[S];  // raw: compared where it is used, so the load is not waited for at issue
     };
     auto load_rows = [&](Rows& R, const int c) {
-        const int tb = c * rows + seg * S;
+        const int tb = c * rows + w * S;
 #pragma unroll
         for (int i = 0; i < S; ++i) {
             const unsigned e = (unsigned)min(tb + i, T - 1) * (unsigned)B + (unsigned)bl;
@@ -174,7 +160,7 @@ __global__ void __launch_bounds__(MAXT, MINB) vtrace_lane_kernel(const VtArgs a)
         for (int i = 0; i <= S; ++i) R.vv[i] = __ldg(a.v + (unsigned)min(tb + i, T) * (unsigned)B + (unsigned)bl);
     };
     auto process = [&](Rows& R, const int c) {
-        const int tb = c * rows + seg * S;  // first step of this thread's segment
+        const int tb = c * rows + w * S;  // first step of this thread's segment
         // ---- 2. per-step terms and the zero-carry scan of this segment
         float rho[S], disc[S], fa[S], g[S], lp2a[S];
 #pragma unroll
@@ -225,9 +211,8 @@ __global__ void __launch_bounds__(MAXT, MINB) vtrace_lane_kernel(const VtArgs a)
             P[i] = prod;
         }
         // ---- 3. exchange the composed maps of the segments, find the carry entering this segment.
-        // Inside the CTA: the carry entering segment s is  A_s + Pm_s * x  with x the carry entering
-        // the CTA's LAST segment; composing all nw maps gives the CTA's own map.  Across the cluster:
-        // x comes from composing the maps of the later CTAs on top of the previous chunk's carry.
+        // The carry entering segment s is  A_s + Pm_s * x  with x the carry entering the LAST segment
+        // (the previous chunk's carry); composing all nw maps gives the carry this chunk passes on.
         const int par = c & 1;
         s_map[par][w][lane] = make_float2(acc[0], P[0]);
         __syncthreads();
@@ -238,21 +223,8 @@ __global__ void __launch_bounds__(MAXT, MINB) vtrace_lane_kernel(const VtArgs a)
             cA = fmaf(q.y, cA, q.x);
             cP = q.y * cP;
         }
-        float x = chunk_carry;
-        if (csize > 1) {
-            if (w == 0) s_cta[par][lane] = make_float2(cA, cP);
-            cluster.sync();
-            float xm = x;
-            for (int r = csize - 1; r >= 0; --r) {
-                if (r == crank) xm = x;
-                const float2 q = *cluster.map_shared_rank(&s_cta[par][lane], r);
-                x = fmaf(q.y, x, q.x);
-            }
-            chunk_carry = x;  // accumulator at the first step of this chunk
-            x = xm;
-        } else {
-            chunk_carry = fmaf(cP, x, cA);
-        }
+        const float x = chunk_carry;
+        chunk_carry = fmaf(cP, x, cA);
         const float mine = fmaf(mineP, x, mineA);
 
         // ---- 4. fix-up, outputs, loss terms
@@ -360,7 +332,6 @@ __global__ void __launch_bounds__(MAXT, MINB) vtrace_lane_kernel(const VtArgs a)
             if (tid == 0) *a.counter = 0u;
         }
     }
-    if (csize > 1) cluster.sync();  // no CTA leaves while a peer may still read its shared memory
 }
 
 int pick_ap(int A) {
@@ -373,24 +344,21 @@ int pick_ap(int A) {
 
 bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
 
-template <int AP, int S, int MAXT, int MINB, bool WITH_LOSS>
-int launch_s(const VtArgs& a, bool vec, unsigned groups, int nw, int cl, cudaStream_t st) {
-    const cudaError_t e =
-        vec ? impala_launch_cl(vtrace_lane_kernel<AP, S, MAXT, MINB, WITH_LOSS, true>, groups * cl, 32 * nw, 0, st, true, false, cl, a)
-            : impala_launch_cl(vtrace_lane_kernel<AP, S, MAXT, MINB, WITH_LOSS, false>, groups * cl, 32 * nw, 0, st, true, false, cl, a);
-    if (e != cudaSuccess) return (int)e;
+template <int AP, int S, bool WITH_LOSS>
+int launch_s(const VtArgs& a, bool vec, unsigned groups, int nw, cudaStream_t st) {
+    if (vec)
+        vtrace_lane_kernel<AP, S, WITH_LOSS, true><<<groups, 32 * nw, 0, st>>>(a);
+    else
+        vtrace_lane_kernel<AP, S, WITH_LOSS, false><<<groups, 32 * nw, 0, st>>>(a);
     return impala_launch_status();
 }
 
-constexpr int kMaxCluster = 8;  // portable cluster size
-
-// Steps per thread (S), warps per CTA (nw) and CTAs per cluster (cl); wide action sets trade S for
-// registers.  Measured on B200 (scripts/tune_vtrace.py, ncu): S = 2; up to 10 segments (T <= 20) one CTA
-// holds the whole unroll in one chunk; longer unrolls walk chunks of 8 x S steps with 8 warps per CTA
-// (T = 100, B = 8192: 17.4 us).  Spreading the segments of a long unroll over a thread-block cluster
-// (DSMEM carry exchange, cl = 4 / 8) works but measured SLOWER - 34-42 us at T = 100, B = 8192: the
-// cluster barriers cost more than the chunk loop they replace - so cl = 1 unless overridden.
-// IMPALA_VTRACE_S / IMPALA_VTRACE_NSEG (warps per CTA) / IMPALA_VTRACE_CLUSTER override the choice.
+// Steps per thread (S) and warps per CTA (nw); the widest action set trades S for registers.
+// Measured on B200 (ncu): S = 2; up to 10 segments (T <= 20) one CTA holds the whole unroll in one
+// chunk; longer unrolls walk chunks of 8 x S steps with 8 warps per CTA (T = 100, B = 8192: 17.4 us).
+// Spreading the segments of a long unroll over a thread-block cluster (DSMEM carry exchange, 4 or 8
+// CTAs) was measured SLOWER - 34-42 us at T = 100, B = 8192: the cluster barriers cost more than
+// the chunk loop they replace.
 template <bool WITH_LOSS>
 int launch(VtArgs& a, cudaStream_t st) {
     if (a.T < 1 || a.B < 1 || a.A < 1) return IMPALA_ERR_BAD_ARG;
@@ -401,29 +369,13 @@ int launch(VtArgs& a, cudaStream_t st) {
     const unsigned groups = (unsigned)((a.B + 31) / 32);
     const bool vec = a.A == AP && aligned16(a.cur_logits) && aligned16(a.beh_logits) &&
                      (!WITH_LOSS || aligned16(a.dlogits));
-    int S = AP == 16 ? 1 : 2;
-    const int s_env = impala_env_int("IMPALA_VTRACE_S", 0);
-    if (AP <= 4 && (s_env == 1 || s_env == 2 || s_env == 5)) S = s_env;
-    const int max_w = S == 5 ? 10 : (AP <= 4 && S == 1 ? kMaxSeg : 16);
+    const int S = AP == 16 ? 1 : 2;
     const int nseg = (a.T + S - 1) / S;
-    const int cl_env = impala_env_int("IMPALA_VTRACE_CLUSTER", 0);
-    const int cl = (cl_env >= 1 && cl_env <= kMaxCluster) ? cl_env : 1;
-    int nw = (nseg + cl - 1) / cl;
-    if (cl == 1 && nw > 10) nw = 8;  // chunk loop: 8 warps per CTA measured best for long unrolls
-    if (nw > max_w) nw = max_w;
-    const int n_env = impala_env_int("IMPALA_VTRACE_NSEG", 0);
-    if (n_env >= 1 && n_env <= max_w) nw = n_env;
-#define VT_AP(APV)                                                                                      \
-    if (AP == APV) {                                                                                    \
-        if (S == 5) return launch_s<APV, 5, 320, 1, WITH_LOSS>(a, vec, groups, nw, cl, st);             \
-        if (S == 1) return launch_s<APV, 1, 1024, 1, WITH_LOSS>(a, vec, groups, nw, cl, st);            \
-        return launch_s<APV, 2, 512, 1, WITH_LOSS>(a, vec, groups, nw, cl, st);                         \
-    }
-    VT_AP(2)
-    VT_AP(4)
-#undef VT_AP
-    if (AP == 8) return launch_s<8, 2, 512, 1, WITH_LOSS>(a, vec, groups, nw, cl, st);
-    return launch_s<16, 1, 512, 1, WITH_LOSS>(a, vec, groups, nw, cl, st);
+    const int nw = nseg <= 10 ? nseg : 8;
+    if (AP == 2) return launch_s<2, 2, WITH_LOSS>(a, vec, groups, nw, st);
+    if (AP == 4) return launch_s<4, 2, WITH_LOSS>(a, vec, groups, nw, st);
+    if (AP == 8) return launch_s<8, 2, WITH_LOSS>(a, vec, groups, nw, st);
+    return launch_s<16, 1, WITH_LOSS>(a, vec, groups, nw, st);
 }
 
 }  // namespace
@@ -446,7 +398,7 @@ extern "C" int impala_vtrace(const float* cur_logits, const float* beh_logits,
 
 extern "C" int64_t impala_vtrace_loss_workspace(int T, int B, int A) {
     if (T < 1 || B < 1 || A < 1) return IMPALA_ERR_BAD_ARG;
-    const int64_t grid = (((int64_t)B + 31) / 32) * kMaxCluster;  // one row per CTA, clusters of up to 8 per group
+    const int64_t grid = ((int64_t)B + 31) / 32;  // one row per CTA
     return grid * 4 * (int64_t)sizeof(double) + 16;  // per-CTA sums + arrival counter
 }
 

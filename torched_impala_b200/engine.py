@@ -27,6 +27,7 @@ ever waits for the previous step.
 """
 from __future__ import annotations
 
+import contextlib
 import ctypes as C
 
 import numpy as np
@@ -43,17 +44,6 @@ _TORCH_DT = {np.float32: torch.float32, np.int32: torch.int32, np.uint8: torch.u
 
 def _ptr(t: torch.Tensor) -> C.c_void_p:
     return C.c_void_p(t.data_ptr())
-
-
-class _NoCtx:
-    def __enter__(self):
-        return self
-
-    def __exit__(self, *exc):
-        return False
-
-
-_NO_CTX = _NoCtx()
 
 
 class LearnerEngine:
@@ -166,28 +156,25 @@ class LearnerEngine:
         buf = world * slot                              # LL elements per parity buffer
         if ok:
             try:
-                for name, nbytes in (("gather", 2 * 16 * buf),):
-                    ptr, handle = C.c_void_p(), (C.c_char * 64)()
-                    _cabi.check(lib.impala_peer_alloc(nbytes, C.byref(ptr), handle), "impala_peer_alloc")
-                    mine[name] = (ptr.value, bytes(handle.raw))
+                ptr, handle = C.c_void_p(), (C.c_char * 64)()
+                _cabi.check(lib.impala_peer_alloc(2 * 16 * buf, C.byref(ptr), handle), "impala_peer_alloc")
+                mine["gather"] = (ptr.value, bytes(handle.raw))
             except Exception as e:  # noqa: BLE001 - reported below, all ranks fall back together
                 ok, err = False, repr(e)
         handles = [None] * world
         dist.all_gather_object(handles, {k: v[1] for k, v in mine.items()} if ok else None, group=self.pg)
         ok = ok and all(h is not None for h in handles)
-        ptrs = {"gather": []}
-        opened = []
+        gather_ptrs, opened = [], []
         if ok:
             try:
                 for r, h in enumerate(handles):
-                    for name in ("gather",):
-                        if r == rank:
-                            ptrs[name].append(mine[name][0])
-                        else:
-                            ptr = C.c_void_p()
-                            _cabi.check(lib.impala_peer_open(h[name], C.byref(ptr)), f"impala_peer_open(rank {r})")
-                            opened.append(ptr.value)
-                            ptrs[name].append(ptr.value)
+                    if r == rank:
+                        gather_ptrs.append(mine["gather"][0])
+                    else:
+                        ptr = C.c_void_p()
+                        _cabi.check(lib.impala_peer_open(h["gather"], C.byref(ptr)), f"impala_peer_open(rank {r})")
+                        opened.append(ptr.value)
+                        gather_ptrs.append(ptr.value)
             except Exception as e:  # noqa: BLE001
                 ok, err = False, repr(e)
         agree = torch.tensor([1 if ok else 0], device=self.dev)
@@ -199,9 +186,7 @@ class LearnerEngine:
             return
         i64 = dict(dtype=torch.int64, device=self.dev)
         fused = bool(lib.impala_mlp_backward_pair_push_supported(self.M_pi, self.M_vf, self.O, self.H_pi, self.H_v, self.A))
-        if os.environ.get("IMPALA_PUSH_FUSED", "1") == "0":
-            fused = False
-        self.peer = dict(gather=mine["gather"][0], opened=opened, gather_ptrs=torch.tensor(ptrs["gather"], **i64),
+        self.peer = dict(gather=mine["gather"][0], opened=opened, gather_ptrs=torch.tensor(gather_ptrs, **i64),
                          seq=torch.zeros(1, **i64), rank=rank, slot=slot, buf=buf, fused=fused,
                          err=torch.zeros(1, dtype=torch.int32, device=self.dev),
                          timeout_s=float(os.environ.get("IMPALA_PEER_TIMEOUT_S", "600")))
@@ -265,16 +250,17 @@ class LearnerEngine:
         for name, _ in _BATCH_FIELDS:
             np.copyto(self.h_views[slot][name], batch[name])
 
-    def ingest(self, slot: int = 0) -> None:
-        """Async H2D of pinned slab `slot` into device slab `slot` on the copy stream."""
+    def _copy_to_slab(self, slot: int, fn: str, *args) -> None:
+        """lib.<fn>(device slab `slot`, *args, copy stream), ordered after the step that last read the slab."""
         cs = self.copy_stream
         if self._slab_used[slot]:
-            cs.wait_event(self.slab_free[slot])  # the step that last read this slab is done
-        _cabi.check(self.lib.impala_ingest(_ptr(self.d_slabs[slot]),
-                                           C.c_void_p(self.h_slabs[slot].data_ptr()),
-                                           self.slab_bytes, C.c_void_p(cs.cuda_stream)),
-                    "impala_ingest")
+            cs.wait_event(self.slab_free[slot])
+        _cabi.check(getattr(self.lib, fn)(_ptr(self.d_slabs[slot]), *args, C.c_void_p(cs.cuda_stream)), fn)
         self.slab_ready[slot].record(cs)
+
+    def ingest(self, slot: int = 0) -> None:
+        """Async H2D of pinned slab `slot` into device slab `slot` on the copy stream."""
+        self.ingest_from(self.h_slabs[slot].data_ptr(), slot)
 
     def register_host(self, address: int, nbytes: int) -> None:
         """Page-lock caller-owned host memory (e.g. a shared-memory trajectory ring) for DMA."""
@@ -285,23 +271,13 @@ class LearnerEngine:
     def ingest_from(self, host_address: int, slot: int = 0) -> None:
         """Like `ingest`, but the source slab is caller-owned (registered) host memory in the
         same batch layout - the DMA reads the actors' shared-memory slab directly."""
-        cs = self.copy_stream
-        if self._slab_used[slot]:
-            cs.wait_event(self.slab_free[slot])
-        _cabi.check(self.lib.impala_ingest(_ptr(self.d_slabs[slot]), C.c_void_p(host_address),
-                                           self.slab_bytes, C.c_void_p(cs.cuda_stream)), "impala_ingest")
-        self.slab_ready[slot].record(cs)
+        self._copy_to_slab(slot, "impala_ingest", C.c_void_p(host_address), self.slab_bytes)
 
     def ingest_shard_from(self, host_address: int, b0: int, B_total: int, slot: int = 0) -> None:
         """Data-parallel ingest: columns [b0, b0 + B_local) of a caller-owned (registered) host slab
         laid out for B_total columns -> device slab `slot` (impala_ingest_shard)."""
-        cs = self.copy_stream
-        if self._slab_used[slot]:
-            cs.wait_event(self.slab_free[slot])
-        _cabi.check(self.lib.impala_ingest_shard(_ptr(self.d_slabs[slot]), C.c_void_p(host_address), self.T, B_total,
-                                                 self.O, self.A, b0, self.B, C.c_void_p(cs.cuda_stream)),
-                    "impala_ingest_shard")
-        self.slab_ready[slot].record(cs)
+        self._copy_to_slab(slot, "impala_ingest_shard", C.c_void_p(host_address), self.T, B_total, self.O, self.A,
+                           b0, self.B)
 
     def load_device_batch(self, batch: dict, slot: int = 0) -> None:
         """Convenience for kernel-only timing: put a batch in HBM and wait for it."""
@@ -404,7 +380,7 @@ class LearnerEngine:
         import threading
 
         if self._loop_thread is not None and self._loop_thread == threading.get_ident():
-            return _NO_CTX
+            return contextlib.nullcontext()
         return torch.cuda.stream(self.stream)
 
     def step(self, slot: int = 0) -> None:
